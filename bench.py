@@ -2,6 +2,7 @@
 """bench.py -- Gaussians/s fwd+bwd of the rasterizer hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|cpu] [--workload c1|c2|c3|c4|c5|mg]
+                    [--dump-outputs DIR]
 
 A "step" = forward + backward of every view of the workload over one synthetic Gaussian cloud (SURVEY.md 8(d)):
 default workload c3 = BASELINE.json configs[2]: 500k Gaussians, 4 views 256x256, RGB + 32 feature channels.
@@ -45,6 +46,56 @@ SH_DEGREE = 1
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+DUMP_MAX_BYTES = 64_000_000
+DUMP_SAMPLE = 65_536  # per-Gaussian rows written for larger clouds
+
+
+def dump_outputs(path, P, arrays, per_gaussian):
+    """Writes every array as <path>/<name>.npy, float64 kept and everything else as float32, so that the outputs of two
+    builds of the project can be compared one for one.  `per_gaussian` arrays have the Gaussian index on axis 0; for clouds
+    of more than DUMP_SAMPLE Gaussians only a fixed, seeded sample of those rows is written, their indices as
+    gaussian_index.npy.  Fails rather than write more than DUMP_MAX_BYTES in all."""
+    def host(x):
+        x = x.detach().cpu().numpy() if hasattr(x, "detach") else np.asarray(x)
+        return x if x.dtype == np.float64 else x.astype(np.float32)
+    out = {k: host(v) for k, v in arrays.items()}
+    idx = slice(None)
+    if P > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(P, DUMP_SAMPLE, replace=False))
+        out["gaussian_index"] = idx.astype(np.float64)
+    for k, v in per_gaussian.items():
+        v = host(v)
+        assert v.shape[0] == P, (k, v.shape)
+        out[k] = np.ascontiguousarray(v[idx])
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the limit of {DUMP_MAX_BYTES}")
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+    log(f"[bench] wrote {len(out)} arrays, {total} bytes, to {path}")
+
+
+def view_outputs(impl, outs):
+    """outs: (R, colour, feature, radii[, depth]) of every view.  Returns them as the caller receives them, stacked over
+    views: colour [V,3,H,W], feature [V,F,H,W], depth [V,H,W], and radii as [P,V] (per Gaussian)."""
+    import torch
+    st = lambda xs, dim=0: torch.stack(list(xs), dim)
+    arrays = {"color": st(o[1] for o in outs)}
+    if impl.name == "reference":  # the build's padded feature width, depth in channel F (RefImpl)
+        feats = [o[2][:impl.F] for o in outs]
+        depths = [o[2][impl.F] for o in outs]
+    else:
+        feats = [o[2] for o in outs]
+        depths = [o[4] for o in outs] if impl.depth else []
+    if impl.F:
+        arrays["feature"] = st(feats)
+    if impl.depth:
+        arrays["depth"] = st(depths)
+    return arrays, {"radii": st((o[3] for o in outs), 1)}
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -253,9 +304,11 @@ def run_step(impl, G, C, T, flat, acc, dist=None, streams=None):
     flat.zero_()
     Rs = 0
     if not streams:
+        images = []
         for cam, ct in zip(C, T):
             out = impl.fwd(G, cam)
             grads = impl.bwd(G, cam, out, ct)
+            images.append(out[:4] + out[7:])
             Rs += int(out[0])
             gd = dict(zip(GRAD_ORDER, grads))
             for k, v in acc.items():
@@ -277,6 +330,8 @@ def run_step(impl, G, C, T, flat, acc, dist=None, streams=None):
             for k, v in acc.items():
                 gd[k].record_stream(main)
                 v.add_(gd[k].reshape(v.shape))
+        images = [out[:4] + out[7:] for out, _ in results]
+    G["last_images"] = images  # (R, colour, feature, radii[, depth]) of every view, for --dump-outputs
     if dist is not None:
         dist.all_reduce(flat)
     return Rs
@@ -649,6 +704,8 @@ def main_dyna(a, wl, base, cfg, torch, rank, world):
     e1.record()
     torch.cuda.synchronize()
     t_stop = time.perf_counter()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, P, {"loss": loss}, {"grad_" + k: v.grad for k, v in L.items() if v.requires_grad})
     clocks = sampler.stop(t_start, t_stop)
     ms_step = e0.elapsed_time(e1) / a.steps
     units = P * 2 * V
@@ -855,7 +912,11 @@ def main():
     ap.add_argument("--no-clocks", action="store_true", help="do not poll nvidia-smi during the run")
     ap.add_argument("--no-stage-timing", action="store_true", help="do not bracket stages with CUDA events")
     ap.add_argument("--streams", type=int, default=4, help="CUDA streams over which independent views are enqueued (ours only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed "
+                    "(images, radii, per-Gaussian gradients; a seeded sample of rows for large clouds) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = dict(WORKLOADS[a.workload])
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -881,6 +942,8 @@ def main():
         if not torch.cuda.is_available() or util.load_reference(32 if need > 3 else 3) is None:
             use_cpu = True
     if use_cpu:
+        if a.dump_outputs:
+            raise SystemExit("--dump-outputs needs a GPU arm: the CPU arm times a sample of views sized by its own speed")
         if rank != 0:
             return 0
         cb, best = cpu_baseline(wl)
@@ -959,6 +1022,11 @@ def main():
     e1.record()
     barrier()
     t_stop = time.perf_counter()
+    if a.dump_outputs and rank == 0:
+        last = [o[:4] + o[7:] for o in G["last_outs"]] if streams and a.impl == "ours" else G["last_images"]
+        arrays, per_gaussian = view_outputs(impl, last)
+        per_gaussian.update(acc)  # the per-Gaussian gradients summed over the views (all-reduced over the ranks)
+        dump_outputs(a.dump_outputs, P, arrays, per_gaussian)
     hs = sorted((b_ - a_) * 1e3 for a_, b_ in zip([t_start] + step_marks[:-1], step_marks))
     meas["host_step_ms"] = {"min": round(hs[0], 3), "median": round(hs[len(hs) // 2], 3), "max": round(hs[-1], 3)}
     if G.get("last_outs") is not None and streams and a.impl == "ours":
@@ -1055,7 +1123,7 @@ def main():
         # drop this workload's device tensors first: the c5 cloud is twice the size
         del G, C, T, flat, acc
         torch.cuda.empty_cache()
-        c5 = strong_scaling_c5(torch, dist, rank, world, max(5, a.steps // 4), a.warmup)
+        c5 = strong_scaling_c5(torch, dist, rank, world, a.steps, a.warmup)
 
     if rank != 0:
         if dist is not None:

@@ -1,7 +1,5 @@
 """CPU tests of the oracle (oracle/gs_oracle.c): internal consistency, a finite-difference check of its backward
 against its own forward (independent of any GPU), and the golden vectors produced by the compiled reference."""
-import glob
-import json
 import os
 
 import numpy as np
@@ -97,42 +95,35 @@ def test_backward_matches_finite_differences(field, gname):
     assert np.linalg.norm(num - ana) <= tol * max(np.linalg.norm(ana), 1e-3), (field, num, ana)
 
 
-GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "g[0-9]*.npz")))
-
-
-@pytest.mark.skipif(not GOLDEN, reason="tests/golden/*.npz not generated yet (tests/golden/make_golden.py on a B200)")
-@pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p)[:-4] for p in GOLDEN])
+@pytest.mark.skipif(not util.REFERENCE_GOLDEN, reason="tests/golden/*.npz not generated yet (tests/golden/make_golden.py on a B200)")
+@pytest.mark.parametrize("path", util.REFERENCE_GOLDEN, ids=[os.path.basename(p)[:-4] for p in util.REFERENCE_GOLDEN])
 def test_oracle_against_reference_golden(path):
     """The restatement vs outputs of the unmodified reference run on a B200 (oracle/_ref)."""
-    z = np.load(path)
-    kw = json.loads(bytes(z["recipe"]).decode())
-    if "bg" in kw:
-        kw["bg"] = tuple(kw["bg"])
-    inp = util.make_inputs(**kw)
+    inp, ref, ref_bw = util.load_reference_golden(path)
     fw, bw = _run(inp)
     F = inp["F"]
     # integer / index outputs: bit-exact
-    assert np.array_equal(fw["radii"], z["fw_radii"])
-    assert np.array_equal(fw["tiles_touched"], z["fw_tiles_touched"])
-    assert fw["num_rendered"] == int(z["fw_num_rendered"])
-    assert np.array_equal(fw["point_list"], z["fw_point_list"])
-    assert np.array_equal(fw["point_list_keys"] >> np.uint64(32), z["fw_point_list_keys"] >> np.uint64(32))  # tile ids
-    assert np.array_equal(fw["ranges"], z["fw_ranges"])
-    assert (fw["n_contrib"] != z["fw_n_contrib"]).mean() <= 1e-3
-    live = z["fw_radii"] > 0
+    assert np.array_equal(fw["radii"], ref["radii"])
+    assert np.array_equal(fw["tiles_touched"], ref["tiles_touched"])
+    assert fw["num_rendered"] == ref["num_rendered"]
+    assert np.array_equal(fw["point_list"], ref["point_list"])
+    assert np.array_equal(fw["point_list_keys"] >> np.uint64(32), ref["point_list_keys"] >> np.uint64(32))  # tile ids
+    assert np.array_equal(fw["ranges"], ref["ranges"])
+    assert (fw["n_contrib"] != ref["n_contrib"]).mean() <= 1e-3
+    live = ref["radii"] > 0
     # floating point: 1e-4 relative L2 (BASELINE.json north_star); depth key bits differ only by FMA contraction
     for k in ("depths", "means2D", "conic_opacity", "cov3D"):
-        if k == "cov3D" and kw.get("precomp_cov"):
+        if k == "cov3D" and inp["g"]["cov3D_precomp"] is not None:
             continue
-        assert util.rel_l2(fw[k][live], z["fw_" + k][live]) < 1e-5, k
-    if not kw.get("precomp_colors"):
-        assert util.rel_l2(fw["rgb"][live], z["fw_rgb"][live]) < 1e-5
-        assert np.array_equal(fw["clamped"][live], z["fw_clamped"][live])
-    assert util.rel_l2(fw["out_color"], z["fw_out_color"]) < 1e-4
+        assert util.rel_l2(fw[k][live], ref[k][live]) < 1e-5, k
+    if inp["g"]["colors_precomp"] is None:
+        assert util.rel_l2(fw["rgb"][live], ref["rgb"][live]) < 1e-5
+        assert np.array_equal(fw["clamped"][live], ref["clamped"][live])
+    assert util.rel_l2(fw["out_color"], ref["out_color"]) < 1e-4
     if F:
-        assert util.rel_l2(fw["out_feature"], z["fw_out_feature"]) < 1e-4
-    assert util.rel_l2(fw["final_T"], z["fw_final_T"]) < 1e-4
+        assert util.rel_l2(fw["out_feature"], ref["out_feature"]) < 1e-4
+    assert util.rel_l2(fw["final_T"], ref["final_T"]) < 1e-4
     for k, v in bw.items():
         if k == "dL_dconic" or (k == "dL_dfeature" and not F):
             continue
-        assert util.rel_l2(v, z["bw_" + k]) < 1e-4, (k, util.rel_l2(v, z["bw_" + k]))
+        assert util.rel_l2(v, ref_bw[k]) < 1e-4, (k, util.rel_l2(v, ref_bw[k]))

@@ -1,10 +1,13 @@
 """GPU parity tests (run with `-m gpu` on the B200 box).  They call the product path through the C ABI
 (include/mgs_rasterizer.h via manigaussian_b200.rasterizer) and compare it with
   (1) the CPU oracle oracle/gs_oracle.c on the same seeded inputs, stage by stage, and
-  (2) the compiled, unmodified reference rasterizer in oracle/_ref when that build travelled with the snapshot.
+  (2) the unmodified reference rasterizer: its stored outputs in tests/golden/, and the compiled reference in oracle/_ref
+      where that build is present.
 Bars (BASELINE.json north_star): tile ids / sort keys / ranges / radii bit-exact; images and all gradient tensors
 within 1e-4 relative L2.
 """
+import os
+
 import numpy as np
 import pytest
 
@@ -35,13 +38,14 @@ def _live(fw):
     return fw["radii"] > 0
 
 
-def check_stagewise_vs_oracle(inp, grad_tol=TOL):
+def check_stagewise_vs_oracle(inp, grad_tol=TOL, scale_modifier=1.0, **kw):
     """Ours vs the C oracle.  Integer stages are checked exactly by feeding OUR upstream outputs to the oracle's
-    downstream stage (so the FMA-contraction difference of the projection cannot leak into an index compare)."""
+    downstream stage (so the FMA-contraction difference of the projection cannot leak into an index compare).
+    `kw` (prefiltered, debug) goes to our path only: the oracle has no such settings."""
     import ctypes as C
     from oracle import gs_oracle as O
-    ours, ours_bw = util.run_ours(inp)
-    orc, orc_bw = util.run_oracle(inp)
+    ours, ours_bw = util.run_ours(inp, scale_modifier=scale_modifier, **kw)
+    orc, orc_bw = util.run_oracle(inp, scale_modifier=scale_modifier)
     P, W, H, F = inp["P"], inp["W"], inp["H"], inp["F"]
     # -- projection: floats by tolerance, integer outputs identical except for documented borderline cases
     live = _live(ours) & _live(orc)
@@ -108,12 +112,7 @@ def test_vs_oracle(name):
     check_stagewise_vs_oracle(util.make_inputs(**CASES[name]), ORACLE_GRAD_TOL.get(name, TOL))
 
 
-@pytest.mark.parametrize("name", list(CASES))
-def test_vs_compiled_reference(name):
-    inp = util.make_inputs(**CASES[name])
-    ref, ref_bw = util.run_reference(inp)
-    if ref is None:
-        pytest.skip("oracle/_ref not built (reference sources are only available in the build container)")
+def check_vs_reference(inp, ref, ref_bw):
     ours, ours_bw = util.run_ours(inp)
     F = inp["F"]
     # bit-exact: everything that decides tile ids and sort keys
@@ -138,6 +137,27 @@ def test_vs_compiled_reference(name):
         if k == "dL_dcolors" and inp["g"]["colors_precomp"] is None:
             pass  # internal gradient in the SH path; still comparable
         assert util.rel_l2(ours_bw[k], ref_bw[k]) < TOL, (k, util.rel_l2(ours_bw[k], ref_bw[k]))
+
+
+@pytest.mark.parametrize("name", list(CASES))
+def test_vs_compiled_reference(name):
+    """Without the reference build: the same bars against the recorded values (util.PARITY_RECORD)."""
+    inp = util.make_inputs(**CASES[name])
+    ref, ref_bw = util.run_reference(inp)
+    if ref is not None:
+        check_vs_reference(inp, ref, ref_bw)
+        return
+    ours, ours_bw = util.run_ours(inp)
+    report = util.compare_with_record("parity_" + name, *util.parity_fields(ours, ours_bw, inp["F"]))
+    bad = {k: v for k, v in report.items() if not v < TOL}
+    assert not bad, (bad, report)
+
+
+@pytest.mark.parametrize("path", util.REFERENCE_GOLDEN, ids=[os.path.basename(p)[:-4] for p in util.REFERENCE_GOLDEN])
+def test_vs_reference_golden(path):
+    """The same bars against stored outputs of the unmodified reference (tests/golden/make_golden.py), so that the
+    comparison with the reference needs no reference build."""
+    check_vs_reference(*util.load_reference_golden(path))
 
 
 def test_depth_plane_matches_feature_channel():

@@ -1,7 +1,9 @@
 """Shared helpers for the parity tests: run the CUDA product path, the CPU oracle (oracle/gs_oracle.c) and,
 when its build travelled with the snapshot, the compiled reference (oracle/_ref) on the same seeded inputs and
 return everything as numpy so tests compare stage by stage."""
+import glob
 import importlib.util
+import json
 import os
 import sys
 
@@ -67,6 +69,96 @@ def load_reference_package(F):
     sys.modules[name] = pkg
     spec.loader.exec_module(pkg)
     return pkg
+
+
+# outputs of the unmodified reference rasterizer, run on a B200 by tests/golden/make_golden.py
+REFERENCE_GOLDEN = sorted(glob.glob(os.path.join(ROOT, "tests", "golden", "g[0-9]*.npz")))
+
+
+def load_reference_golden(path):
+    """(inputs, forward dict, backward dict) of one stored reference run, in the layout of run_reference().  Entries of
+    culled Gaussians in the per-Gaussian float state are zero (the reference leaves them uninitialised)."""
+    z = np.load(path)
+    kw = json.loads(bytes(z["recipe"]).decode())
+    if "bg" in kw:
+        kw["bg"] = tuple(kw["bg"])
+    fw = {k[3:]: z[k] for k in z.files if k.startswith("fw_")}
+    fw["num_rendered"] = int(fw["num_rendered"])
+    bw = {k[3:]: z[k] for k in z.files if k.startswith("bw_")}
+    return make_inputs(**kw), fw, bw
+
+
+# --------------------------------------------------------------------------- recorded parity values
+# Expected values of the reference comparisons at sizes whose outputs are far too large to store (tests/golden/
+# make_parity_record.py): a SHA-256 digest of every array compared bit for bit, and of every tensor compared by relative
+# L2 its exact norm plus a CountSketch, which is linear, so that ||sketch(a) - sketch(b)|| estimates ||a - b|| over the
+# whole tensor (within about 25 % at 64 buckets, ample for a 1e-4 bar met at 1e-5; a single wrong entry is caught exactly).
+PARITY_RECORD = os.path.join(ROOT, "tests", "golden", "parity_record.npz")
+SKETCH_BUCKETS = 64
+_RECORD = {}
+
+
+def sketch(x, k=SKETCH_BUCKETS):
+    x = np.asarray(x, np.float64).ravel()
+    rng = np.random.default_rng(x.size)
+    bucket = rng.integers(0, k, x.size, dtype=np.int32)
+    sign = rng.integers(0, 2, x.size, dtype=np.int8) * 2 - 1
+    return np.bincount(bucket, weights=x * sign, minlength=k)
+
+
+def _sha(x):
+    import hashlib
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(x).tobytes()).digest(), np.uint8)
+
+
+def summarize(exact, close, values=None):
+    """exact: arrays compared bit for bit; close: tensors compared by relative L2; values: scalars kept as they are."""
+    s = {"sha_" + k: _sha(v) for k, v in exact.items()}
+    for k, v in close.items():
+        s["norm_" + k] = np.float64(np.linalg.norm(np.asarray(v, np.float64)))
+        s["sketch_" + k] = sketch(v).astype(np.float32)
+    s.update({"value_" + k: np.float64(v) for k, v in (values or {}).items()})
+    return s
+
+
+def parity_fields(fw, bw, F, depth=False):
+    """What the reference comparisons look at (test_parity_gpu.check_vs_reference): (bit-exact arrays, rel-L2 tensors).
+    n_contrib is bit-exact too: its mismatch bar (1e-5 of the pixels) admits no mismatch at these image sizes."""
+    live = fw["radii"] > 0
+    exact = {k: fw[k] for k in ("radii", "tiles_touched", "point_list_keys", "point_list", "ranges", "n_contrib")}
+    exact.update({k: fw[k][live].view(np.uint32) for k in ("depths", "means2D", "conic_opacity")})
+    exact["num_rendered"] = np.int64(fw["num_rendered"])
+    close = {"out_color": fw["out_color"], "final_T": fw["final_T"]}
+    if F:
+        close["out_feature"] = fw["out_feature"]
+    if depth:
+        close["out_depth"] = fw["out_depth"]
+    close.update({k: v for k, v in bw.items() if not (k == "dL_dfeature" and not F)})
+    return exact, close
+
+
+def load_record(name):
+    if not _RECORD:
+        z = np.load(PARITY_RECORD)
+        for key in z.files:
+            case, field = key.split("/", 1)
+            _RECORD.setdefault(case, {})[field] = z[key]
+    assert name in _RECORD, f"{name} is not in {PARITY_RECORD}"
+    return _RECORD[name]
+
+
+def compare_with_record(name, exact, close):
+    """Asserts the digests of `exact` equal the recorded ones; returns the estimated relative L2 of every `close` tensor."""
+    rec = load_record(name)
+    assert sorted(exact) == sorted(k[4:] for k in rec if k.startswith("sha_")), name
+    assert sorted(close) == sorted(k[5:] for k in rec if k.startswith("norm_")), name
+    for k, v in exact.items():
+        assert np.array_equal(_sha(v), rec["sha_" + k]), f"{name}: {k} differs from the recorded value"
+    report = {}
+    for k, v in close.items():
+        d, n = float(np.linalg.norm(sketch(v) - rec["sketch_" + k])), float(rec["norm_" + k])
+        report[k] = d / n if n > 0 else d
+    return report
 
 
 def _obtain(base_ptr, off, nbytes, align=128):
@@ -136,11 +228,11 @@ def _t(x, dev="cuda"):
 
 
 # --------------------------------------------------------------------------- oracle
-def run_oracle(inp, backward=True):
+def run_oracle(inp, backward=True, scale_modifier=1.0):
     from oracle import gs_oracle as O
     cam, g, ct = inp["cam"], inp["g"], inp["ct"]
     kw = dict(scales=g["scales"], rotations=g["rotations"], cov3D_precomp=g["cov3D_precomp"], shs=g["shs"],
-              sh_degree=g["sh_degree"], colors_precomp=g["colors_precomp"], feature=g["feature"])
+              sh_degree=g["sh_degree"], colors_precomp=g["colors_precomp"], feature=g["feature"], scale_modifier=scale_modifier)
     fw = O.forward(g["means3D"], g["opacities"], cam["viewmatrix"], cam["projmatrix"], cam["campos"], inp["W"], inp["H"],
                    cam["tanfovx"], cam["tanfovy"], inp["bg"], **kw)
     bw = None
